@@ -2,7 +2,7 @@
 """Headline benchmark: tokens/sec of one Long-VITA prefill forward (ViT tower + projector + 48-layer
 14B decoder + masked LM head) on synthetic frames, through the HF `forward()` surface.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--frames F]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--frames F] [--dump-outputs DIR]
 
 A "step" is one full prefill of the configured prompt.  N = 1: BASELINE.json configs[1]
 ("Long-VITA-16K bf16 single B200, 64 synthetic frames -> 16K tokens").  Launched under torchrun
@@ -315,7 +315,13 @@ def main():
                     help="minutes-per-step configs (1M tokens): honour --warmup < 3 and skip the separate e2e pass; "
                          "the printed line is then marked as outside the timing contract")
     ap.add_argument("--layers", type=int, default=None, help="debug: fewer decoder layers (number is then INVALID)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (the last-position logits) to DIR/logits.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl b200 (the reference arm times a sample and computes no outputs)")
     # stdout carries exactly ONE JSON line: everything libraries print meanwhile (e.g. NCCL's
     # "NCCL version ..." banner, written to fd 1 from C) is routed to stderr until the line is emitted
     sys.stdout.flush()
@@ -468,12 +474,26 @@ def main():
     timer = ops.KernelTimer()
     ops.set_kernel_timer(timer)
     n0 = ops.launch_count()
-    ms_resident = timed(lambda: forward_resident(images_d, ids_d, idx_d), args.steps)
+    last = {}
+
+    def step_resident():
+        last["logits"] = forward_resident(images_d, ids_d, idx_d)
+
+    ms_resident = timed(step_resident, args.steps)
     log(f"timed region done: {ms_resident / args.steps:.1f} ms/step")
     launches = ops.launch_count() - n0
     ops.set_kernel_timer(None)
     torch.cuda.synchronize()
     ksum = timer.summary()
+    if args.dump_outputs and rank == 0:
+        # copied now: later forwards (the e2e pass) may reuse the buffer the logits live in
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        import numpy as np
+
+        logits = last["logits"].float().cpu().numpy()
+        np.save(os.path.join(args.dump_outputs, "logits.npy"), logits)
+        log(f"wrote {args.dump_outputs}/logits.npy {logits.shape} float32")
+    del last
     # e2e: host buffers, H2D + forward + D2H inside the timed region
     if args.long_run:
         ms_e2e = None

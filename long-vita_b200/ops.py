@@ -212,7 +212,8 @@ def attention(q, k, v, *, causal: bool, scale: Optional[float] = None):
 
 
 def _sm_count(device) -> int:
-    return torch.cuda.get_device_properties(device).multi_processor_count if torch.cuda.is_available() else 148
+    """SMs of `device`; a B200's 148 for tensors that are not on a GPU (the host tests' oracle-backed operators)."""
+    return torch.cuda.get_device_properties(device).multi_processor_count if torch.device(device).type == "cuda" else 148
 
 
 def attention_decode(q: torch.Tensor, k_cache: torch.Tensor, v_cache: torch.Tensor, length: int, *,

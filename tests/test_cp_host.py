@@ -129,30 +129,32 @@ def _sync_worker(rank, world, port):
     dist.init_process_group("gloo", rank=rank, world_size=world)
     try:
         from oracle import ref_loader
+        from tests.util import digest, recorded
 
         cfg, ids, idx = _prompt(5, world)
         S = ids.shape[1]
         sh = CP.shard_prompt(ids, idx, world, rank, 256)
-        gen = ref_loader.load_megatron_generation(world, rank, dist.group.WORLD)
         # per-token "logits" [b, s_local, 3] of this rank's shard, as forward_step hands them to sync_output
         local = torch.stack([sh.input_ids[0].float(), sh.position_ids.float(), sh.position_ids.float() * 2], dim=-1).unsqueeze(0)
-        full = gen.sync_output(local)
-        assert full.shape == (1, S, 3)
-        assert torch.equal(full[0, :, 1], torch.arange(S).float())                  # global order restored
-        assert torch.equal(full[0, :, 0], ids[0].float())
+
+        def run():
+            return digest(ref_loader.load_megatron_generation(world, rank, dist.group.WORLD).sync_output(local))
+
+        full = recorded(f"sync_output_cp{world}", run, store=rank == 0)      # every rank receives the same sequence
+        pos = torch.arange(S).float()
+        assert full == digest(torch.stack([ids[0].float(), pos, pos * 2], dim=-1).unsqueeze(0))   # global order restored
         # ... which is what zigzag_unpermute_index does with a plain concatenation of the shards
         gathered = [torch.empty_like(local) for _ in range(world)]
         dist.all_gather(gathered, local)
-        assert torch.equal(torch.cat(gathered, dim=1)[:, CP.zigzag_unpermute_index(S, world)], full)
+        assert digest(torch.cat(gathered, dim=1)[:, CP.zigzag_unpermute_index(S, world)]) == full
     finally:
         dist.destroy_process_group()
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="/root/reference not mounted (GPU box)")
 def test_references_own_sync_output_restores_global_order_from_our_shards():
-    """Live, 2 ranks over gloo: the reference's inference-side gather (generation.py:542-566, executed from
-    /root/reference) applied to the shards cp.shard_prompt produced returns the sequence in global order, and
-    equals cp.zigzag_unpermute_index on the concatenated shards."""
+    """2 ranks over gloo: the reference's inference-side gather (generation.py:542-566; a recorded run of it) applied
+    to the shards cp.shard_prompt produced returns the sequence in global order, and equals
+    cp.zigzag_unpermute_index on the concatenated shards."""
     with socket.socket() as s:
         s.bind(("127.0.0.1", 0))
         port = s.getsockname()[1]

@@ -1,8 +1,9 @@
 """Pin the CPU oracle (tests are CPU-only).
 
 The reference ships no tests or golden vectors, so the oracle is pinned against
-  (1) golden outputs generated from the reference's OWN code run in the build container
-      (tests/golden/make_golden.py; regenerated and compared live when /root/reference is mounted):
+  (1) golden outputs generated from the reference's OWN code (tests/golden/make_golden.py, and the outputs the
+      tests below store in tests/golden/ref_recorded.pt when run with LV_RECORD_GOLDEN=1 where the reference's
+      sources are present - oracle/ref_loader.py):
       InternVisionModel / ResamplerProjector / pixel_shuffle, and the WHOLE LongVITAForCausalLM.forward
       (vision tower -> projector -> embedding scatter -> Qwen2 decoder -> norm -> lm_head),
   (2) the installed third-party modules whose arithmetic the reference delegates to
@@ -22,6 +23,7 @@ from long_vita_b200.weights import synthetic_state_dict
 from oracle import model as OM
 from oracle import ops as O
 from oracle import ref_loader
+from tests.util import digest, recorded
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 sys.path.insert(0, GOLD)
@@ -41,8 +43,9 @@ def test_vit_and_projector_match_reference_golden():
     assert hashlib.sha256(images.view(torch.int16).numpy().tobytes()).hexdigest() == gold["images_sha256"]
     vit = OM.vit_forward(cfg, w, images.float())
     proj = OM.projector_forward(cfg, w, vit[:, 1:, :])
+    proj_s = proj[:, gold["proj_rows"]]                   # the fixture keeps two of every three projector rows
     assert torch.allclose(vit, gold["vit_out"], rtol=1e-4, atol=1e-4), float((vit - gold["vit_out"]).abs().max())
-    assert torch.allclose(proj, gold["proj_out"], rtol=1e-4, atol=1e-4)
+    assert torch.allclose(proj_s, gold["proj_out"], rtol=1e-4, atol=1e-4)
 
 
 def test_pixel_shuffle_matches_reference_golden_bit_exact():
@@ -50,11 +53,19 @@ def test_pixel_shuffle_matches_reference_golden_bit_exact():
     assert torch.equal(O.pixel_shuffle_half(gold["x"]), gold["y"])
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="/root/reference not mounted (GPU box)")
 def test_live_reference_modules_agree_with_golden_files():
-    ref = ref_loader.load()
+    """A recorded run of the reference's pixel_shuffle reproduces the committed fixture, and on a second geometry
+    (odd batch, wider channels) agrees with the oracle bit for bit."""
     gold = torch.load(os.path.join(GOLD, "ref_pixel_shuffle.pt"))
-    assert torch.equal(ref.pixel_shuffle(gold["x"], 0.5), gold["y"])
+    x2 = torch.arange(3 * 4 * 4 * 10, dtype=torch.int32).reshape(3, 4, 4, 10)
+
+    def run():
+        ref = ref_loader.load()
+        return {"y": ref.pixel_shuffle(gold["x"], 0.5).clone(), "y2": ref.pixel_shuffle(x2, 0.5).clone()}
+
+    r = recorded("pixel_shuffle", run)
+    assert torch.equal(r["y"], gold["y"])
+    assert torch.equal(O.pixel_shuffle_half(x2), r["y2"])
 
 
 def _sha(t):
@@ -96,33 +107,53 @@ def test_whole_model_oracle_matches_the_references_own_forward():
     assert abs(float(want) - float(gold["loss"])) < 1e-4
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="/root/reference not mounted (GPU box)")
 def test_live_reference_forward_reproduces_the_whole_model_golden():
+    """A recorded run of the reference's forward reproduces the committed last-8 logits; its logits of every position
+    (num_logits_to_keep = 0), at four of the fixture's sampled rows, match the oracle's full forward."""
     gold, cfg, w, ids, images, idx = _long_vita_golden()
-    model = ref_loader.build_reference_long_vita(cfg, w)
-    with torch.no_grad():
-        out = model(input_ids=ids, images=images, image_indices=idx, num_logits_to_keep=8)
-    assert torch.allclose(out.logits[0], gold["logits_last8"], rtol=1e-5, atol=1e-5)
+    rows = gold["rows"][::4]
+
+    def run():
+        model = ref_loader.build_reference_long_vita(cfg, w)
+        with torch.no_grad():
+            last8 = model(input_ids=ids, images=images, image_indices=idx, num_logits_to_keep=8).logits[0]
+            full = model(input_ids=ids, images=images, image_indices=idx).logits[0]
+        return {"logits_last8": digest(last8), "logits_rows": full[rows].clone()}
+
+    r = recorded("long_vita_forward", run)
+    assert r["logits_last8"] == digest(gold["logits_last8"])
+    logits = OM.long_vita_forward(cfg, w, ids, images, idx)[0]
+    assert torch.allclose(logits[rows], r["logits_rows"], rtol=2e-4, atol=2e-4), float((logits[rows] - r["logits_rows"]).abs().max())
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="/root/reference not mounted (GPU box)")
 def test_live_reference_cp_function_reproduces_the_shard_golden():
+    """A recorded run of the reference's get_batch_on_this_cp_rank reproduces the committed shards."""
     from make_golden import cp_golden_prompt
 
     gold = torch.load(os.path.join(GOLD, "ref_cp_shards.pt"))
     ids, idx = cp_golden_prompt()
     S = ids.shape[1]
-    for (cp, r), want in list(gold["shards"].items())[:3]:
-        mod, cpu_placement = ref_loader.load_megatron_training_utils(cp, r, S)
-        batch = {"tokens": ids.clone(), "position_ids": torch.arange(S).unsqueeze(0),
-                 "external_images": torch.arange(idx.shape[1]).view(-1, 1).clone(), "external_indices": idx.clone(),
-                 "attention_mask": None}
-        with cpu_placement():
-            b = mod.get_batch_on_this_cp_rank(batch)
+
+    def run():
+        out = {}
+        for (cp, r) in list(gold["shards"])[:3]:
+            mod, cpu_placement = ref_loader.load_megatron_training_utils(cp, r, S)
+            batch = {"tokens": ids.clone(), "position_ids": torch.arange(S).unsqueeze(0),
+                     "external_images": torch.arange(idx.shape[1]).view(-1, 1).clone(), "external_indices": idx.clone(),
+                     "attention_mask": None}
+            with cpu_placement():
+                b = mod.get_batch_on_this_cp_rank(batch)
+            out[(cp, r)] = {k: None if v is None else digest(v) for k, v in b.items()}
+        assert torch.arange(3, device="cpu").device.type == "cpu" and torch.tensor([1]).sum() == 1   # patches were undone
+        return out
+
+    got = recorded("cp_shards", run)
+    assert list(got) == list(gold["shards"])[:3]
+    for (cp, r), b in got.items():
+        want = gold["shards"][(cp, r)]
         assert set(b) == set(want)
         for k, v in want.items():
-            assert (v is None and b[k] is None) or torch.equal(b[k], v), (cp, r, k)
-    assert torch.arange(3, device="cpu").device.type == "cpu" and torch.tensor([1]).sum() == 1   # patches were undone
+            assert (v is None and b[k] is None) or b[k] == digest(v), (cp, r, k)
 
 
 def test_oracle_full_forward_equals_the_references_incremental_decoding():
@@ -303,19 +334,22 @@ def test_whole_model_oracle_runs_and_uses_image_features():
     assert not torch.allclose(a, b) and not torch.allclose(a, c)
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="/root/reference not mounted (GPU box)")
 def test_live_megatron_vision_downsample_matches_oracle_bit_exact():
     """The Megatron twin of the projector's front end - MegatronVisionModel.forward_downsample / pixel_shuffle
-    (long_vita_megatron/pretrain_long_vita.py:467-483, 572-582), executed from /root/reference: drop the class
-    token, view as [n, 32, 32, C], pixel-shuffle x0.5."""
+    (long_vita_megatron/pretrain_long_vita.py:467-483, 572-582), a recorded run of the reference's code: drop the
+    class token, view as [n, 32, 32, C], pixel-shuffle x0.5."""
     import types
 
-    m = ref_loader.load_class_methods("long_vita_megatron/pretrain_long_vita.py", "MegatronVisionModel",
-                                      {"forward_downsample", "pixel_shuffle"})
-    me = types.SimpleNamespace(add_class_token=True, vision_downsample_ratio=0.5, vision_downsample_stride=1)
-    me.pixel_shuffle = lambda x, scale_factor=0.5: m["pixel_shuffle"](me, x, scale_factor)
     x = torch.arange(2 * 17 * 6, dtype=torch.int32).reshape(2, 17, 6)               # 1 class token + 4 x 4 patches
-    want = m["forward_downsample"](me, x)
+
+    def run():
+        m = ref_loader.load_class_methods("long_vita_megatron/pretrain_long_vita.py", "MegatronVisionModel",
+                                          {"forward_downsample", "pixel_shuffle"})
+        me = types.SimpleNamespace(add_class_token=True, vision_downsample_ratio=0.5, vision_downsample_stride=1)
+        me.pixel_shuffle = lambda x, scale_factor=0.5: m["pixel_shuffle"](me, x, scale_factor)
+        return m["forward_downsample"](me, x).clone()
+
+    want = recorded("megatron_vision_downsample", run)
     got = O.pixel_shuffle_half(x[:, 1:].reshape(2, 4, 4, 6)).reshape(2, 4, 24)
     assert torch.equal(got, want)
 
@@ -383,20 +417,23 @@ def test_siglip_tower_matches_transformers_siglip_encoder():
     assert torch.allclose(out, ref, rtol=1e-4, atol=1e-4), float((out - ref).abs().max())
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="/root/reference not mounted (GPU box)")
 def test_live_megatron_local_rmsnorm_matches_oracle_bit_exact():
     """a5: the reference's Megatron-local RMSNorm (core/transformer/custom_layers/transformer_engine.py:54-79:
-    `_norm(x.float()).type_as(x) * weight`), executed from /root/reference, against oracle.ops.rmsnorm in bf16."""
+    `_norm(x.float()).type_as(x) * weight`), a recorded run of the reference's code, against oracle.ops.rmsnorm in bf16."""
     import types
 
-    m = ref_loader.load_class_methods("long_vita_megatron/core/transformer/custom_layers/transformer_engine.py", "RMSNorm",
-                                      {"_norm", "forward"})
     g = torch.Generator().manual_seed(2)
     x = (torch.randn(37, 640, generator=g) * 3).to(torch.bfloat16)
     w = (1 + 0.1 * torch.randn(640, generator=g)).to(torch.bfloat16)
-    me = types.SimpleNamespace(eps=1e-6, weight=w)
-    me._norm = lambda t: m["_norm"](me, t)
-    assert torch.equal(m["forward"](me, x), O.rmsnorm(x, w, 1e-6))
+
+    def run():
+        m = ref_loader.load_class_methods("long_vita_megatron/core/transformer/custom_layers/transformer_engine.py", "RMSNorm",
+                                          {"_norm", "forward"})
+        me = types.SimpleNamespace(eps=1e-6, weight=w)
+        me._norm = lambda t: m["_norm"](me, t)
+        return digest(m["forward"](me, x))
+
+    assert recorded("megatron_local_rmsnorm", run) == digest(O.rmsnorm(x, w, 1e-6))
 
 
 # ---- frame preprocessing (SURVEY.md 8f-4): Pillow's fixed-point bicubic resize + normalisation ----
@@ -415,8 +452,8 @@ def test_frame_preprocessing_oracle_matches_the_references_own_process_images_fi
 
 
 def test_frame_preprocessing_oracle_matches_the_reference_live_at_448():
-    if not ref_loader.available():
-        pytest.skip("/root/reference is not mounted")
+    """The reference's ImageProcessor.process_images at the real 448 size (a recorded run: the digest of each output,
+    which is too large to store) against the oracle, bit for bit."""
     import sys
 
     import numpy as np
@@ -427,9 +464,12 @@ def test_frame_preprocessing_oracle_matches_the_reference_live_at_448():
     from oracle import preprocess as P
 
     rng = np.random.default_rng(7)
-    for h, w in [(360, 640), (500, 333), (448, 448), (100, 100), (448, 600)]:
-        f = rng.integers(0, 256, (2, h, w, 3), dtype=np.uint8)
-        assert np.array_equal(P.process_frames(list(f)), reference_process_images(f, 448).numpy()), (h, w)
+    shapes = [(360, 640), (500, 333), (448, 448), (100, 100), (448, 600)]
+    frames = [rng.integers(0, 256, (2, h, w, 3), dtype=np.uint8) for h, w in shapes]
+    want = recorded("process_images_448", lambda: [digest(reference_process_images(f, 448).numpy()) for f in frames])
+    assert len(want) == len(frames)
+    for f, d in zip(frames, want):
+        assert digest(P.process_frames(list(f))) == d, f.shape
     # the product's host-side coefficient tables (long_vita_b200/preprocess.py) are the oracle's
     from long_vita_b200 import preprocess as PP
 
@@ -455,10 +495,8 @@ def test_dynamic_tiling_oracle_matches_the_references_own_process_dynamic_fixtur
 
 
 def test_dynamic_tiling_oracle_matches_the_reference_live_at_448():
-    """The same comparison live, at the real tile size, including a grid that is narrower than the image on one axis
-    and wider on the other."""
-    if not ref_loader.available():
-        pytest.skip("/root/reference is not mounted")
+    """The same comparison at the real tile size, including a grid that is narrower than the image on one axis and
+    wider on the other (a recorded run of the reference: grid and digest of each output)."""
     import numpy as np
 
     sys.path.insert(0, GOLD)
@@ -467,9 +505,18 @@ def test_dynamic_tiling_oracle_matches_the_reference_live_at_448():
     from oracle import preprocess as P
 
     rng = np.random.default_rng(5)
-    for h, w in ((500, 700), (1300, 400), (448, 448), (600, 2100)):
-        im = rng.integers(0, 256, (h, w, 3), dtype=np.uint8)
-        ref, gref = reference_process_dynamic(im, 448)
+    images = [rng.integers(0, 256, (h, w, 3), dtype=np.uint8) for h, w in ((500, 700), (1300, 400), (448, 448), (600, 2100))]
+
+    def run():
+        out = []
+        for im in images:
+            ref, gref = reference_process_dynamic(im, 448)
+            out.append((tuple(int(x) for x in gref), digest(ref.numpy())))
+        return out
+
+    want = recorded("process_dynamic_448", run)
+    assert len(want) == len(images)
+    for im, (gref, d) in zip(images, want):
         got, grid = P.process_dynamic(im, 1, 12, 448)
-        assert grid == tuple(int(x) for x in gref), (h, w)
-        assert np.array_equal(got, ref.numpy()), (h, w)
+        assert grid == gref, im.shape
+        assert digest(got) == d, im.shape

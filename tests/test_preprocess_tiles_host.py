@@ -1,7 +1,7 @@
 """Dynamic-patch tiling of still images (SURVEY.md 8f-4, image_processor.py:263-285, 404-448) - CPU side.
 
 * the product's grid chooser (`long_vita_b200.preprocess.dynamic_tile_grid`, host arithmetic) against the reference's own
-  `dynamic_preprocess` (live, when /root/reference is mounted), the oracle and the committed fixture;
+  `dynamic_preprocess` (a recorded run, tests/golden/ref_recorded.pt), the oracle and the committed fixture;
 * the per-element bodies of the CUDA kernels (`csrc/preprocess_core.h`, the text the kernels compile) built with gcc
   and driven with the product's own tables and grid: bit-identical bf16 tiles to the reference fixture.
 The kernels themselves (launch geometry, device pointers) are the business of tests/test_gpu_preprocess.py.
@@ -22,7 +22,7 @@ sys.path.insert(0, ROOT)
 
 from long_vita_b200 import preprocess as PP          # noqa: E402
 from oracle import preprocess as OP                  # noqa: E402
-from oracle import ref_loader                        # noqa: E402
+from tests.util import recorded                      # noqa: E402
 
 
 def _sizes():
@@ -44,15 +44,15 @@ def test_tile_grid_equals_the_oracle_and_the_fixture():
         assert (gx * S, gy * S) == tuple(gp)
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="/root/reference not mounted")
 def test_tile_grid_equals_the_references_own_dynamic_preprocess():
     sys.path.insert(0, GOLD)
     from make_golden import reference_dynamic_grid
 
-    for w, h in _sizes():
-        assert PP.dynamic_tile_grid(w, h, 1, 12, 448) == reference_dynamic_grid(w, h, 448, 1, 12), (w, h)
-    for w, h in _sizes()[:40]:
-        assert PP.dynamic_tile_grid(w, h, 1, 6, 336) == reference_dynamic_grid(w, h, 336, 1, 6), (w, h)
+    cases = [(w, h, 448, 1, 12) for w, h in _sizes()] + [(w, h, 336, 1, 6) for w, h in _sizes()[:40]]
+    want = recorded("dynamic_grid", lambda: [tuple(reference_dynamic_grid(w, h, S, lo, hi)) for w, h, S, lo, hi in cases])
+    assert len(want) == len(cases)
+    for (w, h, S, lo, hi), grid in zip(cases, want):
+        assert PP.dynamic_tile_grid(w, h, lo, hi, S) == grid, (w, h, S)
 
 
 def test_vectorised_resampling_tables_equal_the_oracle_loop():
