@@ -170,7 +170,9 @@ __device__ __forceinline__ uint4 ld_peer_v4(const void* p) {
 // 2^x on the FMA pipe (no MUFU): round-to-nearest split x = n + f, f in [-0.5, 0.5], cubic minimax for 2^f
 // (max relative error 7.5e-5, tools/exp2_poly.py - 50x below the bf16 rounding P gets anyway), exponent
 // add through the low mantissa bits of the magic-number sum.  x is clamped to >= -125 so the result
-// stays a normal number (a masked -inf score becomes 2^-125 ~ 2e-38 instead of 0: invisible in l and P V).
+// stays a normal number: a masked -inf score becomes 2^-125 ~ 2e-38 instead of 0.  That is invisible in l and P V
+// of a row with at least one visible key.  A row that sees no key at all would get l > 0 (2^-125 per polynomial
+// exponential) and the mean of V, so the epilogues test a per-row flag (some visited tile had a finite maximum).
 __device__ __forceinline__ float ex2_poly(float x) {
   x = fmaxf(x, -125.f);
   const float t = x + 12582912.f;            // 1.5 * 2^23: the integer part of x lands in the low mantissa bits
@@ -777,6 +779,7 @@ __global__ void __launch_bounds__(A_THREADS, 1)
         if (jd < j_mask) j_mask = (int)jd;
       }
       float m_used = 0.f, l = 0.f;
+      bool seen = false;   // some visited tile holds a visible key of this row
       for (int j = 0; j < n; ++j) {
         int g = j;         // global key tile of this step (context parallelism visits them out of order)
         if (CP) g = walk.next(cpp);
@@ -826,6 +829,7 @@ __global__ void __launch_bounds__(A_THREADS, 1)
           mx[c] = fmaxf(mx[c], __uint_as_float(s[c * 16 + 15]));
         }
         const float mx_all = fmax3(fmax3(mx[0], mx[1], mx[2]), fmax3(mx[3], mx[4], mx[5]), fmaxf(mx[6], mx[7])) * scale_log2;
+        seen |= mx_all > -INFINITY;
 
         // ---- lazy rescale ----
         if (j == 0) {
@@ -897,7 +901,7 @@ __global__ void __launch_bounds__(A_THREADS, 1)
       }
 
       // ---------------- epilogue: O / l -> bf16 -> smem (swizzled) -> TMA store; LSE ----------------
-      const float inv_l = (n > 0 && l > 0.f) ? 1.f / l : 0.f;
+      const float inv_l = (seen && l > 0.f) ? 1.f / l : 0.f;
       if (n > 0) {
         mbar_wait_a(a_ofull, ocnt & 1);
         ++ocnt;
@@ -935,7 +939,7 @@ __global__ void __launch_bounds__(A_THREADS, 1)
       }
       tc_fence_before();
       if (p.lse != nullptr && w.row0[t] + row < p.sq) {
-        const float lse = (n > 0 && l > 0.f) ? (m_used + log2f(l)) * 0.69314718055994530942f : -INFINITY;
+        const float lse = (seen && l > 0.f) ? (m_used + log2f(l)) * 0.69314718055994530942f : -INFINITY;
         p.lse[((long long)w.b * p.hq + w.h) * p.sq + w.row0[t] + row] = lse;
       }
       fence_proxy_async_smem();
@@ -1225,6 +1229,7 @@ __global__ void __launch_bounds__(A_THREADS, 1)
       const int n = w.n[t];
       const long long qpos = w.qpos[t] + row;
       float m_used = 0.f, l = 0.f;
+      bool seen = false;   // some visited tile holds a visible key of this row
       for (int i = 0; i < n; ++i) {
         const int b = i & 1;
         mbar_wait(&s_full[t * 2 + b], scnt[b] & 1);
@@ -1260,6 +1265,7 @@ __global__ void __launch_bounds__(A_THREADS, 1)
           mx3 = fmax3(mx3, __uint_as_float(s[1][k + 2]), __uint_as_float(s[1][k + 3]));
         }
         const float mx = fmaxf(fmaxf(mx0, mx1), fmaxf(mx2, mx3)) * p.scale_log2;
+        seen |= mx > -INFINITY;
 
         float alpha = 1.f;
         bool rescale = false;
@@ -1313,7 +1319,7 @@ __global__ void __launch_bounds__(A_THREADS, 1)
       }
 
       // ---------------- epilogue ----------------
-      const float inv_l = (n > 0 && l > 0.f) ? 1.f / l : 0.f;
+      const float inv_l = (seen && l > 0.f) ? 1.f / l : 0.f;
       if (n > 0) {
         mbar_wait(&o_done[t], (pv_base + n - 1) & 1);
         pv_base += n;
@@ -1345,7 +1351,7 @@ __global__ void __launch_bounds__(A_THREADS, 1)
       }
       tc_fence_before();
       if (p.lse != nullptr && w.row0[t] + row < p.sq) {
-        const float lse = (n > 0 && l > 0.f) ? (m_used + log2f(l)) * 0.69314718055994530942f : -INFINITY;
+        const float lse = (seen && l > 0.f) ? (m_used + log2f(l)) * 0.69314718055994530942f : -INFINITY;
         p.lse[((long long)w.b * p.hq + w.h) * p.sq + w.row0[t] + row] = lse;
       }
       fence_proxy_async_smem();

@@ -48,6 +48,11 @@ def check(L, b, sq, sk, hq, hkv, d, causal, seed=0, layout="bshd", **kw):
     args = {k_: v_ for k_, v_ in kw.items() if k_ in ("q_seg_len", "q_seg_pos", "kv_pos0")}
     out, lse = L.attention_fwd(qd, kd, vd, causal=causal, layout=layout, return_lse=True, **args)
     out = out.permute(perm)
+    # rows that see no key (causal sq > sk, keys that start after a query's position): exactly 0 and -inf
+    empty = torch.isneginf(lse_ref)
+    lse_empty = lse.cpu()[empty]
+    assert torch.isneginf(lse_empty).all(), lse_empty.unique()[:4]
+    assert not out.cpu()[empty.permute(0, 2, 1)].any()
     e_out, e_total, e_floor = excess_error(out, ref)
     finite = torch.isfinite(lse_ref)
     e_lse = float((lse.cpu()[finite] - lse_ref[finite]).abs().max())
@@ -90,6 +95,12 @@ def test_attention_cross_lengths_bottom_right_causal(L):
     # sk > sq: query i sees keys <= i + (sk - sq)
     check(L, 1, 256, 1024, 4, 2, 128, True, seed=4)
     check(L, 1, 100, 612, 4, 4, 64, True, seed=5)
+    # sq > sk: the first sq - sk query rows see no key, inside a query tile whose other rows do
+    check(L, 1, 300, 200, 4, 2, 128, True, seed=10)
+    check(L, 1, 130, 40, 4, 4, 64, True, seed=11)
+    # keys start at position 940: query rows 0-39 (positions 900-939) see none
+    check(L, 1, 256, 512, 4, 2, 128, True, seed=12, q_seg_pos=(900, 0), kv_pos0=940,
+          q_pos=torch.arange(256) + 900, kv_pos_t=torch.arange(512) + 940)
 
 
 def test_attention_strided_megatron_views(L):

@@ -40,6 +40,8 @@ def run(sq, sk, hq, hkv, d, causal, b=1, seed=0):
         (1025, 1025, 16, 16, 64, False),   # ViT geometry, ragged tiles
         (300, 300, 2, 1, 64, True),
         (128, 640, 2, 2, 128, True),       # bottom-right aligned causal, sk > sq
+        (300, 200, 4, 2, 128, True),       # sq > sk: the first 100 query rows see no key
+        (130, 40, 2, 2, 64, True),         # sq > sk: 90 of the 128 rows of the first query tile see no key
     ],
 )
 def test_attention_backward(lib_built, sq, sk, hq, hkv, d, causal):
@@ -48,6 +50,8 @@ def test_attention_backward(lib_built, sq, sk, hq, hkv, d, causal):
         assert torch.isfinite(a).all(), name
         e = excess(a, r)
         assert e < 3e-3, (name, e, rel_fro(a, r))
+    if causal and sq > sk:
+        assert not dq[:, : sq - sk].any()
 
 
 def test_attention_backward_batch(lib_built):
